@@ -13,6 +13,8 @@ A "step" runs the hot path over `--blocks-per-step` consecutive 20 ms blocks.
   torchrun ... bench.py --gpus N                         channel groups sharded over N GPUs, forward
                                                          transform on rank 0 + one NCCL broadcast of
                                                          the spectrum per step (north_star / SURVEY 8e)
+  python bench.py ... --dump-outputs DIR                 also write the channel outputs of the last timed
+                                                         step to DIR (compare two builds output for output)
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.  The GPU arm never imports the
 oracle: inputs come from ka9q_radio_b200/workloads.py; the parity self-check and the CPU baseline run in subprocesses.
 """
@@ -33,6 +35,9 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+# the tree may be read-only: no bytecode caches next to the sources, here or in the subprocesses
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 METRIC = "input Msamples/s through forward+filter+inverse at N channels"
 L2_BYTES = 126e6   # B200 L2 (B200_PROFILING.md); the resident input a rank cycles through must exceed it
@@ -483,6 +488,8 @@ def run_ours(args) -> None:
     stride = max(1, nchan // 22)
     chans_chk = sorted(set(list(range(0, nchan, stride)) + [nchan - 1] + _tone_channels(w)))
     o_host = out.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, w, cz, o_host)
     pairs = {}
     for b in blocks_chk:
         for c in chans_chk:
@@ -579,6 +586,35 @@ def run_ours(args) -> None:
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname: str, w, cz, o_host: np.ndarray) -> None:
+    """The channel outputs of the last timed step as a caller of the channel bank receives them: for each block of the step,
+    every channel's olen complex samples in channel order -> DIR/outputs.npy, float32 [blocks, samples, 2] (re, im).
+    Outputs larger than DUMP_BYTES (all files together) are sampled with a fixed seed: whole blocks, and whole channels
+    only when one block alone is too large.  DIR/blocks.npy and DIR/channels.npy list what was kept (float64 indices within
+    the step and the workload's channel list).  With several GPUs these are rank 0's channels."""
+    rng = np.random.default_rng(0)
+    nb, n = o_host.shape[0], len(w.channels)
+    olen = np.array([c.olen for c in w.channels])
+    budget = DUMP_BYTES - 8 * (nb + n) - 3 * 128          # the two index files and the three .npy headers
+    chans = np.arange(n)
+    if olen.sum() * 8 > budget:
+        order = rng.permutation(n)
+        chans = np.sort(order[: np.searchsorted(np.cumsum(olen[order]) * 8, budget, side="right")])
+        if chans.size == 0:
+            raise SystemExit(f"--dump-outputs: one channel's block alone exceeds {DUMP_BYTES} bytes")
+    idx = np.concatenate([np.arange(cz.bank.out_offset(c), cz.bank.out_offset(c) + olen[c]) for c in chans])
+    keep = min(nb, budget // (idx.size * 8))
+    blocks = np.arange(nb) if keep == nb else np.sort(rng.choice(nb, keep, replace=False))
+    outs = np.ascontiguousarray(o_host[np.ix_(blocks, idx)]).view(np.float32).reshape(len(blocks), idx.size, 2)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "outputs.npy"), outs)
+    np.save(os.path.join(dirname, "blocks.npy"), blocks.astype(np.float64))
+    np.save(os.path.join(dirname, "channels.npy"), chans.astype(np.float64))
 
 
 class _Multi:
@@ -737,7 +773,7 @@ def run_e2e_filter_h(args, w, host: np.ndarray) -> dict:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=None, choices=["cfg2", "cfg3", "cfg4", "cfg5"],
@@ -759,7 +795,14 @@ def main():
                          "egress and HBM bound it); `spectrum-mc` = the same through this repository's NVSwitch-multicast copy kernel; "
                          "`input` = broadcast of the raw window, forward replicated; `slices` = rank 0 scatters per-rank bin slices; "
                          "`a2a` = block-parallel forward + all-to-all of per-rank bin slices")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm: write the channel outputs of the last timed step to DIR/outputs.npy (float32, at most "
+                         "64 MB: a fixed sample of the step's blocks when larger; DIR/blocks.npy and DIR/channels.npy list them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm only times")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

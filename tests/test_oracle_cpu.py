@@ -2,9 +2,10 @@
 
 1. oracle FFT vs numpy/scipy (the DFT contract FFTW3 publishes);
 2. the restatement vs the committed golden fixtures (outputs of the reference's own filter.c);
-3. the restatement vs the reference itself (oracle/_ref) when that library is present;
+3. the restatement vs the reference's own slicing loops, every shift (also golden fixtures);
 4. analytic known-answer tests derived from the reference code paths (SURVEY.md 8c).
 """
+import hashlib
 from pathlib import Path
 
 import numpy as np
@@ -72,42 +73,45 @@ def test_restatement_matches_golden(oracle, name):
 
 
 def test_restatement_matches_reference_library(oracle):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    """Against the reference's own filter.c (tests/golden/reference_library.npz, made by make_golden.py)."""
+    z, _, _ = _golden_case("reference_library")
     L, M = 4800, 1201
     x = oracle.siggen_real(5 * L, 0.2, 0.05, 0.3123, 1.0)
-    assert np.array_equal(x, oracle.ref_siggen_real(5 * L, 0.2, 0.05, 0.3123, 1.0))
+    assert hashlib.sha256(x.tobytes()).digest() == z["x_sha"].tobytes()   # the reference's sig_gen made the same stream
     chans = [dict(olen=48, shift=s, low=-0.3, high=0.4, beta=9.0) for s in (1874, -1874, 0, 2999, -3005, 2990, 12)]
     chans.append(dict(olen=96, shift=1870, low=-0.2, high=0.2, beta=4.0, isb=True))
+    assert np.array_equal(z["chan_params"], [[c["olen"], c["shift"], c["low"], c["high"], c["beta"], c.get("isb", False)]
+                                             for c in chans])
     o1, s1 = oracle.run_stream(x, L, M, chans, notch_bins=[5], keep_spectra=True)
-    o2, s2 = oracle.ref_run_stream(x, L, M, chans, notch_bins=[5], keep_spectra=True)
+    st = int(z["spec_stride"])
     for b in range(5):
-        assert rel_err(s1[b], s2[b]) < 1e-6
+        assert np.abs(s1[b][::st] - z["spec_sub"][b]).max() / z["spec_absmax"][b] < 1e-6
         for c in range(len(chans)):
-            den = max(np.abs(o2[b][c]).max(), 1e-9)
-            assert np.abs(o1[b][c] - o2[b][c]).max() / den < 1e-6
+            o2 = z[f"out{c}"][b]
+            den = max(np.abs(o2).max(), 1e-9)
+            assert np.abs(o1[b][c] - o2).max() / den < 1e-6
 
 
 def test_slice_sweep_matches_reference_library(oracle):
     """Every integer shift, REAL and COMPLEX masters, even and odd slave sizes: the restated
-    slicing equals the reference's loops entry by entry (SURVEY.md 8a probe, re-run here)."""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built")
-    for in_type, L, M in ((oracle.KO_REAL, 480, 121), (oracle.KO_COMPLEX, 480, 121)):
+    slicing equals the reference's loops entry by entry (SURVEY.md 8a probe).  tests/golden/slice_sweep.npz holds the
+    reference's master spectrum, responses and, for every slice it made, the master bin behind each entry (conjugated
+    or not, or none); the reference's slices are rebuilt from those exactly."""
+    z = np.load(GOLD / "slice_sweep.npz")
+    olens = (48, 24, 40)
+    assert np.array_equal(z["olens"], olens)
+    for tag, in_type, L, M in (("real", oracle.KO_REAL, 480, 121), ("complex", oracle.KO_COMPLEX, 480, 121)):
         N = L + M - 1
-        rng = np.random.default_rng(7)
-        x = (rng.standard_normal(L) + (1j * rng.standard_normal(L) if in_type == oracle.KO_COMPLEX else 0))
-        x = x.astype(np.complex64 if in_type == oracle.KO_COMPLEX else np.float32)
-        with oracle.RefSession(L, M, in_type) as s:
-            ids = [s.add_channel(olen, -0.3, 0.3, 8.0) for olen in (48, 24, 40)]
-            s.write(x)
-            X = s.spectrum()
-            lim = N // 2 if in_type == oracle.KO_COMPLEX else N
-            for shift in range(-lim + 1, lim):
-                for i in ids:
-                    _, fd = s.execute(i, shift, want_fdomain=True)
-                    mine = oracle.slice_multiply(in_type, X, s.response(i), shift)
-                    assert np.abs(mine - fd).max() <= 2e-7 * np.abs(fd).max() + 1e-12, (in_type, shift, i)
+        X = z[f"{tag}_X"]
+        lim = N // 2 if in_type == oracle.KO_COMPLEX else N
+        assert len(z[f"{tag}_src0"]) == 2 * lim - 1
+        for i, olen in enumerate(olens):
+            R = z[f"{tag}_R{i}"]
+            assert len(R) == olen * N // L
+            for shift, src in zip(range(-lim + 1, lim), z[f"{tag}_src{i}"]):
+                fd = oracle.rebuild_slice(X, R, src)
+                mine = oracle.slice_multiply(in_type, X, R, shift)
+                assert np.abs(mine - fd).max() <= 2e-7 * np.abs(fd).max() + 1e-12, (in_type, shift, i)
 
 
 def test_analytic_kat_tone_gain(oracle):
